@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Mvoxels/s to converged min-cut (BASELINE.json metric) on the headline workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size S] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size S] [--no-extras] [--dump-outputs DIR]
 
 A "step" is one complete pass of the hot path over one synthetic volume: graph build (n-link stencil, regional
 t-links, markers, solver state -- one fused kernel) -> max-flow to convergence -> mask + energy.  Workload
@@ -23,6 +23,9 @@ boundary_difference_exponential (sigma = RMS neighbour difference), fg ball / bg
              N > 1: config 5 (1024^3) z-slab partitioned over the N GPUs
   cpu_baseline: the reference's BK solver (oracle/_ref, real reference sources) timed on a bounded 256^3 sample of the
              same generator on the host, 1 thread (BK is serial)
+
+`--dump-outputs DIR` writes what the last timed step returned -- energy and mask -- as .npy files (see output_arrays); the
+inputs are generated from a fixed seed, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the reference's CPU path on the SAME 512^3 instance (numpy terms + C++ graph fill + BK maxflow +
 read-out; ~40 s and ~40 GB of host memory per step, so at most 2 steps are measured whatever K says -- stated in the line).
@@ -67,6 +70,7 @@ if ROOT not in sys.path:
 METRIC = "Mvoxels/sec to min-cut"
 UNIT = "Mvoxels/s"
 B_ALG = 11  # algorithmic bytes / voxel of config 3: image 4 + prob 4 + fg 1 + bg 1 + mask 1 (SURVEY.md §8d)
+DUMP_SAMPLE = 1 << 22  # mask voxels --dump-outputs draws (float32 values + float64 indices: 48 MB at most)
 
 
 def measured_peak():
@@ -196,6 +200,25 @@ def cpu_baseline_obj(r, size, workload_size):
         "maxflow_only_value": r["n"] / max(r["maxflow_s"], 1e-9) / 1e6,
         "host_cores_available": os.cpu_count(), "host_cpu_quota": CPU_QUOTA,
     }
+
+
+def output_arrays(energy, mask):
+    """The energy and the mask of one step as the arrays --dump-outputs writes, each to <name>.npy:
+      energy.npy             float64 [1]   the min-cut energy maxflow() returned
+      mask_fg_per_plane.npy  float64 [S0]  foreground voxels per index of the first axis (covers the whole mask)
+      mask_sample.npy        float32 [k]   mask values (1 = foreground) at
+      mask_sample_index.npy  float64 [k]   flat C-order voxel indices: every voxel of a mask of at most DUMP_SAMPLE voxels,
+                                           else the sorted distinct draws of DUMP_SAMPLE uniform indices from a fixed seed"""
+    mask = numpy.asarray(mask)
+    flat = mask.reshape(-1)
+    if flat.size <= DUMP_SAMPLE:
+        idx = numpy.arange(flat.size)
+    else:
+        idx = numpy.unique(numpy.random.default_rng(0).integers(0, flat.size, size=DUMP_SAMPLE))
+    return {"energy": numpy.asarray([energy], dtype=numpy.float64),
+            "mask_fg_per_plane": mask.reshape(mask.shape[0], -1).sum(axis=1, dtype=numpy.int64).astype(numpy.float64),
+            "mask_sample": flat[idx].astype(numpy.float32),
+            "mask_sample_index": idx.astype(numpy.float64)}
 
 
 def committed_mask_hash(key="config3_512"):
@@ -365,6 +388,11 @@ def run_gpu_arm(args):
         csize = args.cpu_size if args.cpu_size else 256
         r = cpu_reference_run(csize)
         out["cpu_baseline"] = cpu_baseline_obj(r, csize, size)
+    if args.dump_outputs:
+        outputs = result["outputs"] if world == 1 else output_arrays(result["energy"], result["mask"])
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            numpy.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -458,6 +486,7 @@ def bench_single(vol, args, torch):
     mask_host = d_mask.cpu().numpy()
     fg_vox = int(mask_host.sum(dtype=numpy.int64))
     mask_hash = sha256_of(mask_host)
+    outputs = output_arrays(energy, mask_host) if args.dump_outputs else None
     del d_mask, mask_host
     value = n / (ms * 1e-3) / 1e6
     launches = int(sum(s["kernel_launches"] for s in stats))
@@ -505,6 +534,7 @@ def bench_single(vol, args, torch):
     del m_e2e, keep
     return {"value": value, "ms_per_step": ms, "clocks": clocks, "e2e": e2e, "gpu_launches": launches,
             "roofline": roof, "roofline_maxflow": roof_mf, "energy": energy, "fg_voxels": fg_vox, "mask_sha256": mask_hash,
+            "outputs": outputs,
             "push_sweeps": stats[-1]["push_sweeps"], "global_relabels": stats[-1]["global_relabels"],
             "relabel_sweeps": stats[-1]["relabel_sweeps"]}
 
@@ -520,7 +550,12 @@ def main():
                     help="edge of the CPU arm's volume; 0 = the workload's own size for --impl reference, 256 for the cpu_baseline object")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip config.extra (configs 2, 4, 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the energy and mask of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_gpu_arm(args)

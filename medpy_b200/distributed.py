@@ -361,7 +361,7 @@ def _slab_resident(shape, rank, world, local_rank, regional, steps, warmup, samp
 def bench_slab(shape, args, rank, world, local_rank):
     """Strong-scaling run of bench.py's workload: the volume is partitioned once, the slab inputs stay resident
     in HBM, each timed step rebuilds the graph, solves and extracts the mask.  Returns the dict bench.py prints
-    (meaningful on rank 0)."""
+    (meaningful on rank 0), with the last timed step's full host mask under "mask" (rank 0; None elsewhere)."""
     import time
     import torch
     import torch.distributed as dist
@@ -422,7 +422,7 @@ def bench_slab(shape, args, rank, world, local_rank):
     roof_mf["ms_per_step"] = None
     return {"value": n / (ms * 1e-3) / 1e6, "ms_per_step": ms, "clocks": r["clocks"], "e2e": e2e,
             "gpu_launches": r["launches"], "roofline": roof, "roofline_maxflow": roof_mf, "energy": energy, "fg_voxels": r["fg_voxels"],
-            "mask_sha256": mask_hash,
+            "mask_sha256": mask_hash, "mask": r["mask"],
             "push_sweeps": s.stats["push_passes"], "global_relabels": s.stats["global_relabels"],
             "relabel_sweeps": s.stats["relabel_rounds"], "sigma": vol["sigma"]}
 

@@ -1,4 +1,4 @@
-"""The reference CLI against the import shim (CPU part) and our own CLI on the GPU."""
+"""MetaImage IO of the import shim (CPU part) and our own CLIs against the oracle on the GPU."""
 import os
 import subprocess
 import sys
@@ -8,7 +8,6 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 COMPAT = os.path.join(ROOT, "medpy_b200", "compat")
-REF_CLI = "/root/reference/bin/medpy_graphcut_voxel.py"
 
 
 def _write_case(tmp_path, shape=(12, 10, 9), ext=".mha"):
@@ -50,25 +49,6 @@ def test_metaimage_roundtrip_and_xyz_order(tmp_path):
             del sys.modules[k]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CLI), reason="reference tree not present")
-def test_reference_cli_runs_unchanged_up_to_the_device(tmp_path):
-    """bin/medpy_graphcut_voxel.py, executed in place and unmodified, imports medpy.* from the shim, parses its
-    arguments, loads the images, splits the markers and reaches graph_from_voxels; without a GPU that is where the
-    product refuses (no CPU fallback); with one it must finish and write the mask."""
-    import torch
-    vol, ip, mp = _write_case(tmp_path)
-    out = str(tmp_path / "out.mha")
-    env = dict(os.environ, PYTHONPATH=COMPAT + os.pathsep + ROOT, PYTHONDONTWRITEBYTECODE="1")
-    r = subprocess.run([sys.executable, REF_CLI, "15.0", ip, mp, out, "--boundary", "diff_exp", "-f"],
-                       env=env, capture_output=True, text=True, timeout=300)
-    if torch.cuda.is_available():
-        assert r.returncode == 0, r.stderr[-2000:]
-        assert os.path.exists(out)
-    else:
-        assert r.returncode != 0
-        assert "no CPU path" in r.stderr or "CUDA" in r.stderr, r.stderr[-2000:]
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("ext", [".mha", ".nii.gz"])
 def test_own_cli_matches_oracle(tmp_path, ext):
@@ -90,9 +70,6 @@ def test_own_cli_matches_oracle(tmp_path, ext):
     assert numpy.array_equal(mask_xyz.T.astype(numpy.uint8), omask)
 
 
-REF_LABEL_CLI = "/root/reference/bin/medpy_graphcut_label.py"
-
-
 def _write_label_case(tmp_path, shape=(12, 10, 9)):
     sys.path.insert(0, COMPAT)
     try:
@@ -111,24 +88,6 @@ def _write_label_case(tmp_path, shape=(12, 10, 9)):
         paths[name] = str(tmp_path / (name + ".mha"))
         save(numpy.ascontiguousarray(arr).T, paths[name], hdr, True)
     return vol, regions, grad, paths
-
-
-@pytest.mark.skipif(not os.path.exists(REF_LABEL_CLI), reason="reference tree not present")
-def test_reference_label_cli_runs_unchanged_up_to_the_device(tmp_path):
-    """bin/medpy_graphcut_label.py in place and unmodified: medpy.filter.relabel, medpy.graphcut.graph_from_labels,
-    energy_label.boundary_stawiaski, what_segment per region and medpy.filter.relabel_map all come from the shim."""
-    import torch
-    vol, regions, grad, paths = _write_label_case(tmp_path)
-    out = str(tmp_path / "out.mha")
-    env = dict(os.environ, PYTHONPATH=COMPAT + os.pathsep + ROOT, PYTHONDONTWRITEBYTECODE="1")
-    r = subprocess.run([sys.executable, REF_LABEL_CLI, paths["grad"], paths["regions"], paths["markers"], out, "-f"],
-                       env=env, capture_output=True, text=True, timeout=300)
-    if torch.cuda.is_available():
-        assert r.returncode == 0, r.stderr[-2000:]
-        assert os.path.exists(out)
-    else:
-        assert r.returncode != 0
-        assert "no CPU" in r.stderr or "CUDA" in r.stderr, r.stderr[-2000:]
 
 
 @pytest.mark.gpu
@@ -154,39 +113,3 @@ def test_own_label_cli_matches_oracle(tmp_path):
     _, rmask, _ = solvers.solve_sparse(int(lab_xyz.max()), i, j, w, wr, tw)
     assert numpy.array_equal(numpy.asarray(mask_xyz).astype(numpy.uint8), rmask[lab_xyz - 1])
 
-
-OTHER_LABEL_CLIS = [
-    ("medpy_graphcut_label_w_regional.py", lambda p, out: [p["grad"], p["regions"], p["markers"], out, "--regional", "atlas",
-                                                            "--radditional", p["atlas"], "--alpha", "0.2", "-f"]),
-    ("medpy_graphcut_label_wsplit.py", lambda p, out: [p["grad"], p["regions"], p["markers"], out, "-f"]),
-]
-# (bin/medpy_graphcut_label_bgreduced.py cannot run on numpy >= 1.13 at all: it subtracts boolean arrays in its own
-#  pre-processing, :217, long before it reaches the graph cut.)
-
-
-@pytest.mark.skipif(not os.path.exists(REF_LABEL_CLI), reason="reference tree not present")
-@pytest.mark.parametrize("script,argv", OTHER_LABEL_CLIS, ids=[c[0] for c in OTHER_LABEL_CLIS])
-def test_other_reference_label_clis_run_unchanged_up_to_the_device(tmp_path, script, argv):
-    """The remaining region-cut scripts of the reference, in place and unmodified: regional_atlas + boundary term
-    (w_regional), graphcut_split(graphcut_stawiaski, ...) (wsplit).
-    Everything they import resolves in the shim; without a GPU they stop where the product refuses to run on a CPU."""
-    import torch
-    sys.path.insert(0, COMPAT)
-    try:
-        from medpy.io import save, Header
-    finally:
-        sys.path.remove(COMPAT)
-    vol, regions, grad, paths = _write_label_case(tmp_path, shape=(24, 22, 20))
-    atlas = (1.0 / (1.0 + numpy.exp(-(vol["image"].astype(numpy.float64) - 50.0) / 15.0))).astype(numpy.float32)
-    paths["atlas"] = str(tmp_path / "atlas.mha")
-    save(numpy.ascontiguousarray(atlas).T, paths["atlas"], Header(spacing=(1.0, 1.0, 1.0), offset=(0.0, 0.0, 0.0)), True)
-    out = str(tmp_path / "out.mha")
-    env = dict(os.environ, PYTHONPATH=COMPAT + os.pathsep + ROOT, PYTHONDONTWRITEBYTECODE="1")
-    r = subprocess.run([sys.executable, os.path.join(os.path.dirname(REF_LABEL_CLI), script)] + argv(paths, out),
-                       env=env, capture_output=True, text=True, timeout=300)
-    if torch.cuda.is_available():
-        assert r.returncode == 0, r.stderr[-2000:]
-        assert os.path.exists(out)
-    else:
-        assert r.returncode != 0
-        assert "no CPU" in r.stderr or "CUDA" in r.stderr, r.stderr[-3000:]

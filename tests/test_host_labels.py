@@ -3,7 +3,6 @@ medpy_b200.graphcut.energy_label / graph_from_labels, the sparse GraphDouble sta
 helpers, and that nothing falls back to a CPU solver."""
 import inspect
 import os
-import re
 import sys
 
 import numpy
@@ -130,46 +129,24 @@ def test_compat_filter_relabel_and_relabel_map():
 
 
 def test_graph_record_and_dimacs_writer_match_the_reference():
-    """medpy.graphcut.Graph + graph_to_dimacs (graph.py:29-265, write.py:27-76) against the unmodified reference."""
+    """medpy.graphcut.Graph + graph_to_dimacs (graph.py:29-265, write.py:27-76) against what the unmodified reference
+    writes and reports for the same graphs (tests/golden/reference_runs_v1.npz)."""
     import io
     from medpy_b200.graphcut import Graph, graph_to_dimacs
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+    try:
+        import make_golden_reference_runs as reference_runs
+    finally:
+        sys.path.pop(0)
 
-    def fill(g):
-        g.set_nodes(5)
-        g.set_nweights({(1, 2): (0.5, 0.25), (2, 3): (1, 0), (4, 5): (0, 2.5)})
-        g.add_tweights({3: (0.1, 0.9), 4: (0, 0)})
-        g.set_source_nodes([1, 2])
-        g.set_sink_nodes([5])
-        return g
-
-    ours = fill(Graph())
+    ours = reference_runs.fill_graph(Graph())
     buf = io.StringIO()
     graph_to_dimacs(ours, buf)
     assert ours.inconsistent() is False
     assert ours.get_nodes() == [1, 2, 3, 4, 5] and ours.get_edges() == [(1, 2), (2, 3), (4, 5)]
     assert ours.get_tweights()[1] == (Graph.MAX, 0) and ours.get_tweights()[5] == (0, Graph.MAX)
-    bad = Graph()
-    bad.set_nodes(2)
-    bad.set_nweights({(1, 2): (1, 1), (2, 1): (1, 1), (1, 3): (1, 1)})
-    bad.set_sink_nodes([7])
-    msgs = bad.inconsistent()
+    msgs = reference_runs.fill_inconsistent(Graph()).inconsistent()
     assert msgs and len(msgs) == 5      # node 7 twice (t-weights, t-nodes), node 3 in an edge, two reversed duplicates
-    if not os.path.isdir("/root/reference/medpy"):
-        return
-    import importlib.util
-    names = {}
-    for mod in ("graph", "write"):
-        src = open("/root/reference/medpy/graphcut/%s.py" % mod).read()
-        src = re.sub(r"^from \.maxflow import .*$", "GraphDouble = None", src, flags=re.M)   # the solver binding is not needed
-        ns = {"__name__": "reference_" + mod}
-        exec(compile(src, mod, "exec"), ns)
-        names[mod] = ns
-    ref = fill(names["graph"]["Graph"]())
-    rbuf = io.StringIO()
-    names["write"]["graph_to_dimacs"](ref, rbuf)
-    assert buf.getvalue() == rbuf.getvalue()
-    rbad = names["graph"]["Graph"]()
-    rbad.set_nodes(2)
-    rbad.set_nweights({(1, 2): (1, 1), (2, 1): (1, 1), (1, 3): (1, 1)})
-    rbad.set_sink_nodes([7])
-    assert sorted(rbad.inconsistent()) == sorted(msgs)
+    z = reference_runs.load()
+    assert buf.getvalue() == reference_runs.text(z, "dimacs")
+    assert "\n".join(sorted(msgs)) == reference_runs.text(z, "inconsistent")

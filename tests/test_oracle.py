@@ -1,6 +1,8 @@
 """CPU tests: the oracle (oracle/energy_terms.py + oracle/bk_lattice.c) against the golden vectors
-produced by the unmodified reference, and against the real reference solver when oracle/_ref exists."""
+produced by the unmodified reference, and against the outputs of the real reference solver and graph builder
+recorded on seeded random inputs (tests/golden/reference_runs_v1.npz)."""
 import os
+import sys
 
 import numpy
 import pytest
@@ -8,6 +10,9 @@ import pytest
 from conftest import golden
 from oracle import energy_terms as et
 from oracle import solvers
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import make_golden_reference_runs as reference_runs  # noqa: E402
 
 NAMES = golden().names()
 
@@ -60,44 +65,32 @@ def test_reference_known_answers():
     assert flow == 3.0 and numpy.array_equal(mask, expect)
 
 
-@pytest.mark.skipif(not solvers.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 def test_port_equals_real_reference_on_random_lattices():
-    rng = numpy.random.default_rng(7)
-    for _ in range(120):
-        nd = int(rng.integers(1, 5))
-        shape = tuple(int(x) for x in rng.integers(1, 7, size=nd))
-        n = int(numpy.prod(shape))
-        wf = [rng.integers(0, 3, size=n).astype(float) for _ in range(nd)]
-        wb = [rng.integers(0, 3, size=n).astype(float) for _ in range(nd)]
-        tr = rng.integers(-3, 4, size=n).astype(float)
-        prob = dict(shape=shape, wf=wf, wb=wb, tr=tr, flow_const=0.0, fg=numpy.zeros(n, numpy.uint8),
-                    bg=numpy.zeros(n, numpy.uint8), src=numpy.maximum(tr, 0), snk=numpy.maximum(-tr, 0))
+    """120 random integer lattices (1-D..4-D): the restatement's flow and mask equal the reference BK's."""
+    z = reference_runs.load()
+    off = 0
+    for k, prob in enumerate(reference_runs.random_lattices()):
         f1, m1, _ = solvers.solve_port(prob)
-        f2, m2, _ = solvers.solve_ref(prob)
-        assert f1 == f2 and numpy.array_equal(m1, m2)
+        m2 = z["lattice/mask"][off:off + m1.size].reshape(m1.shape)
+        off += m1.size
+        assert f1 == z["lattice/flow"][k] and numpy.array_equal(m1, m2), k
+    assert off == z["lattice/mask"].size
 
 
-@pytest.mark.skipif(not solvers.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 def test_port_equals_real_reference_float_32cubed():
-    from medpy_b200 import synthetic
-    vol = synthetic.two_blob_volume((32, 32, 32), seed=0)
-    prob = et.build_problem(vol["fg"], vol["bg"], regional=(vol["prob"], 0.1),
-                            boundary=("difference_exponential", vol["image"], vol["sigma"], False))
-    f1, m1, _ = solvers.solve_port(prob)
-    f2, m2, _ = solvers.solve_ref(prob)
-    assert f1 == f2 and numpy.array_equal(m1, m2)
+    """The bench workload's generator at 32^3 (float64 capacities): flow and mask equal the reference BK's."""
+    z = reference_runs.load()
+    f1, m1, _ = solvers.solve_port(reference_runs.blob32_problem())
+    assert f1 == z["blob32/flow"] and numpy.array_equal(m1, z["blob32/mask"])
     assert 0 < m1.sum() < m1.size
 
 
-@pytest.mark.skipif(not (os.path.isdir("/root/reference/medpy") and solvers.have_ref()), reason="reference tree / pyshim not present")
 def test_voxel_oracle_fuzzed_against_the_live_reference():
     """120 random lattices (1-D..4-D, the eight boundary terms, five image dtypes, random sigma / spacing / regional term /
     overlapping markers) through the reference's own graph_from_voxels: weights, t-links, flow and mask equal the
     restatement's bit for bit; weight <= 0 ValueErrors occur in the same cases
-    (tests/golden/fuzz_voxels_against_reference.py)."""
-    import subprocess
-    import sys
-    script = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fuzz_voxels_against_reference.py")
-    r = subprocess.run([sys.executable, script, "120", "11"], capture_output=True, text=True, timeout=900,
-                       env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
-    assert r.returncode == 0 and "ok 120" in r.stdout, r.stdout[-1500:] + r.stderr[-1500:]
+    (tests/golden/fuzz_voxels_against_reference.py, replayed against the reference's recorded outputs)."""
+    import fuzz_voxels_against_reference as fuzz
+    z = reference_runs.load()
+    cases, seed = reference_runs.VOX_FUZZ
+    fuzz.check(cases, seed, {k[4:]: z[k] for k in z.files if k.startswith("vox/")})

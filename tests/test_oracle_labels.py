@@ -1,7 +1,8 @@
 """The numpy restatement of the label-graph energy terms (oracle/energy_label_terms.py) against what the unmodified
 reference did on the same inputs (tests/golden/golden_labels_v1.npz, made by tests/golden/make_golden_labels.py):
 every set_nweight / set_tweight call, bit for bit and in the reference's order; whole graph_from_labels cuts through
-the real BK solver where oracle/_ref is built."""
+the real BK solver where oracle/_ref is built.  The general-graph BK restatement and the label-term fuzz compare with
+the reference's outputs recorded on seeded inputs (tests/golden/reference_runs_v1.npz)."""
 import os
 import sys
 
@@ -9,8 +10,10 @@ import numpy
 import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
 from oracle import energy_label_terms as elt  # noqa: E402
 from oracle import solvers  # noqa: E402
+import make_golden_reference_runs as reference_runs  # noqa: E402
 
 G = numpy.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_labels_v1.npz"))
 NAMES = [str(n) for n in G["names"]]
@@ -102,36 +105,12 @@ def test_whole_cut_through_reference_bk(nm, tag):
 
 
 # ---- the BK restatement for general graphs (oracle/bk_sparse.c) ------------------------------------------------------
-def _random_graph(rng, n, m, integer):
-    i = rng.integers(0, n, size=m)
-    j = rng.integers(0, n, size=m)
-    keep = i != j
-    i, j = i[keep], j[keep]
-    if integer:
-        cap = rng.integers(0, 20, size=i.size).astype(float)      # zero capacities are legal for sum_edge (graph.h:461)
-        rev = rng.integers(0, 20, size=i.size).astype(float)
-        src = rng.integers(0, 30, size=n).astype(float)
-        snk = rng.integers(0, 30, size=n).astype(float)
-    else:
-        cap = rng.uniform(1e-3, 2.0, size=i.size)
-        rev = rng.uniform(1e-3, 2.0, size=i.size)
-        src = rng.uniform(0, 3.0, size=n)
-        snk = rng.uniform(-0.5, 3.0, size=n)                        # negative t-weights are legal (graph.py:462-498)
-    fg = rng.choice(n, size=max(1, n // 20), replace=False)
-    bg = rng.choice(n, size=max(1, n // 20), replace=False)
-    tw = [(numpy.arange(n), src, snk), (fg, numpy.full(fg.size, 65535.0), numpy.zeros(fg.size)),
-          (bg, numpy.zeros(bg.size), numpy.full(bg.size, 65535.0))]
-    return i, j, cap, rev, tw
-
-
-@pytest.mark.skipif(not solvers.have_ref(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("seed", range(40))
+@pytest.mark.parametrize("seed", reference_runs.SPARSE_SEEDS)
 def test_sparse_port_equals_reference_bk_bit_for_bit(seed):
-    rng = numpy.random.default_rng(1000 + seed)
-    n = int(rng.integers(2, 600))
-    m = int(rng.integers(1, 8 * n))
-    i, j, cap, rev, tw = _random_graph(rng, n, m, seed % 2 == 0)
-    rflow, rmask, _ = solvers.solve_sparse_ref(n, i, j, cap, rev, tw)
+    z = reference_runs.load()
+    n, i, j, cap, rev, tw = reference_runs.sparse_case(seed)
+    before = sum(reference_runs.sparse_case(s)[0] for s in range(seed))
+    rflow, rmask = z["sparse/flow"][seed], z["sparse/mask"][before:before + n]
     pflow, pmask, _ = solvers.solve_sparse_port(n, i, j, cap, rev, tw)
     assert pflow == rflow                      # same arc order => same augmentations => same float64 flow
     assert numpy.array_equal(pmask, rmask)
@@ -161,12 +140,11 @@ def test_sparse_port_reference_diamond():
     assert flow == 4.0 and mask.tolist() == [1, 1, 1, 0]
 
 
-@pytest.mark.skipif(not (os.path.isdir("/root/reference/medpy") and solvers.have_ref()), reason="reference tree / pyshim not present")
 def test_label_oracle_fuzzed_against_the_live_reference():
     """150 random label images (2-D..4-D, five image dtypes, F order, random alpha / directedness): every call the
-    reference issues equals the restatement's, bit for bit (tests/golden/fuzz_labels_against_reference.py)."""
-    import subprocess
-    script = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fuzz_labels_against_reference.py")
-    r = subprocess.run([sys.executable, script, "150", "7"], capture_output=True, text=True, timeout=600,
-                       env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
-    assert r.returncode == 0 and "ok 150" in r.stdout, r.stdout[-1500:] + r.stderr[-1500:]
+    reference issues equals the restatement's, bit for bit (tests/golden/fuzz_labels_against_reference.py, replayed
+    against the reference's recorded calls)."""
+    import fuzz_labels_against_reference as fuzz
+    z = reference_runs.load()
+    cases, seed = reference_runs.LAB_FUZZ
+    fuzz.check(cases, seed, {k[4:]: z[k] for k in z.files if k.startswith("lab/")})
