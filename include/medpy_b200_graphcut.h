@@ -122,6 +122,12 @@ int mgc_trim_pools(void);
  * markers, maxflow, mgc_check).  graph_from_voxels switches it on because it always adds the markers right after the
  * boundary term, which lets the marker upload overlap the stencil kernel. */
 #define MGC_OPT_DEFER_WEIGHT_CHECK 1
+/* MGC_OPT_KEEP_INPUTS (default 0): the caller promises that the DEVICE arrays it passes to mgc_build_voxel_graph stay
+ * valid and unchanged until the next build or mgc_reset on the handle.  This lets the build run lazily on them: blocks
+ * that hold no source excess write only their residual mask and labels, and their capacities are computed again from
+ * the inputs when the solve first reaches them.  Host and strided inputs are staged into the handle's own memory and
+ * never need the promise; without it, caller-owned device inputs get an eager build. */
+#define MGC_OPT_KEEP_INPUTS 2
 int mgc_set_option(mgc_graph* g, int32_t option, int64_t value);
 /* Deliver a deferred verdict now (MGC_OK / MGC_E_WEIGHT). */
 int mgc_check(mgc_graph* g);
@@ -218,6 +224,9 @@ int mgc_get_trcap(mgc_graph* g, int64_t node, double* trcap);
 int mgc_get_node_num(const mgc_graph* g, int64_t* n);
 int mgc_get_arc_num(const mgc_graph* g, int64_t* n);
 int mgc_get_stats(const mgc_graph* g, mgc_stats* out);
+/* Lazy build (MGC_OPT_KEEP_INPUTS, MEDPY_GC_LAZY): build blocks (8 x 8 x 32 voxels) of the last build if it ran lazily, else
+ * 0, and how many of them held their capacity planes at the last maxflow (built hot or materialised on demand). */
+int mgc_get_lazy_stats(const mgc_graph* g, int64_t* build_blocks, int64_t* materialised);
 
 /* ---- pre-step of the boundary_maximum_* terms (SURVEY.md §8 row f1) ----------------------------------- */
 

@@ -158,6 +158,19 @@ struct mgc_graph {
     bool debug_checks = false;         // MEDPY_GC_DEBUG=1: device-side invariant + flow-conservation checks around every solve
     double debug_excess0 = 0.0;        // clamped source excess the solve started from
     bool fuse_build = true;            // mgc_build_voxel_graph uses the single-pass k_build_tile (MEDPY_GC_FUSE=0: four passes)
+    // lazy build (gc_build.cuh, MODE 1): cold 8 x 8 x 32 blocks leave cap / tr / excess unwritten until the push passes
+    // reach them.  bflag[block] = 1 once a block's planes are valid; d_lazy[0] counts such blocks.  The build's inputs,
+    // tensor maps and parameters are kept until every block is materialised, the handle is reset or rebuilt.
+    bool lazy_build = true;            // MEDPY_GC_LAZY=0: always eager
+    bool keep_inputs = false;          // MGC_OPT_KEEP_INPUTS: caller-owned device inputs stay valid until the next build / reset
+    bool lazy = false;                 // the current build left cold blocks behind
+    int* bflag = nullptr;
+    int* d_lazy = nullptr;
+    BuildMaps lazy_maps{};
+    BuildArgs lazy_args{};
+    BoundaryParams lazy_P{};
+    int64_t lazy_blocks = 0;           // build blocks of the last lazy build (0: eager)
+    int64_t lazy_materialised = 0;     // ... of which hold their planes at the last read-out
     int build_chunks = 8;              // host inputs: z-chunks whose upload overlaps the build of the previous chunk
     bool solved = false;
     bool has_nlinks = false;
@@ -573,6 +586,11 @@ int create_impl(int32_t ndim, const int64_t* shape, int64_t z0, int64_t z1, bool
         for (int i = 0; i < 2 && !rc; ++i) { rc = alloc_buf(g, tb, &p); g->rl_items[i] = (int*)p; }
         for (int i = 0; i < 4 && !rc; ++i) { rc = alloc_buf(g, tb, &p); g->pl_items[i >> 1][i & 1] = (int*)p; }
         if (!rc) { rc = alloc_buf(g, 256, &p); g->d_tcount = (int*)p; }
+        if (!rc && !slab) {
+            const size_t nbuild = (size_t)((g->L.dim[0] + 7) / 8) * ((g->L.dim[1] + 7) / 8) * ((g->L.dim[2] + 31) / 32);
+            rc = alloc_buf(g, nbuild * sizeof(int), &p); g->bflag = (int*)p;
+            if (!rc) { rc = alloc_buf(g, 64, &p); g->d_lazy = (int*)p; }
+        }
         {   // dirty-tile tracking for the partial relabel reset (MEDPY_GC_PARTIAL_RESET=0: off)
             const char* ed = getenv("MEDPY_GC_PARTIAL_RESET");
             g->TL.dflag = nullptr; g->TL.ditems = nullptr; g->TL.dcount = nullptr;
@@ -680,6 +698,7 @@ int create_impl(int32_t ndim, const int64_t* shape, int64_t z0, int64_t z1, bool
     if (const char* f0 = getenv("MEDPY_GC_DEBUG")) g->debug_checks = atoi(f0) != 0;
     if (const char* f3 = getenv("MEDPY_GC_FIRST_TEST")) g->skip_first_test = atoi(f3) == 0;
     if (const char* f1 = getenv("MEDPY_GC_FUSE")) g->fuse_build = atoi(f1) != 0;
+    if (const char* f4 = getenv("MEDPY_GC_LAZY")) g->lazy_build = atoi(f4) != 0;
     if (const char* f2 = getenv("MEDPY_GC_CHUNKS")) if (atoi(f2) > 0) g->build_chunks = atoi(f2);
     cudaEventCreateWithFlags(&g->ev_bad, cudaEventDisableTiming);
     for (auto& ev : g->ev_b) cudaEventCreate(&ev);
@@ -1059,12 +1078,18 @@ int relabel_tiles_run(mgc_graph* g, int* any, bool want_any = true)
     return MGC_OK;
 }
 
+int lazy_materialise_list(mgc_graph* g, const WorkList& tiles);
+
 // one colour: consume its current list; still-active tiles go to its alternate list, receivers of cross-face flow
 // to the list the other colour consumes next
 int push_color(mgc_graph* g, int color)
 {
     g->flow_started = true;
     const int a = g->pl_sel[color], oa = g->pl_sel[1 - color];
+    if (g->lazy && g->nd == 3) {          // every block the listed tiles can write into holds its capacity planes
+        int rc = lazy_materialise_list(g, pl(g, color, a));
+        if (rc) return rc;
+    }
     CK(cudaMemsetAsync(cursor(g), 0, sizeof(int), g->stream));
     if (g->nd == 4) {
         k_push_tile4<double><<<g->n_ctas, T4_VOX, 0, g->stream>>>(g->L, g->TL4, g->S, g->smask, g->iters_now, g->pflag, pl(g, color, a),
@@ -1294,7 +1319,10 @@ int readout(mgc_graph* g, double* energy_part)
     g->st.kernel_launches += 2;
     double sc[2] = {0, 0};
     CK(cudaMemcpyAsync(sc, g->d_scalars, sizeof(sc), cudaMemcpyDeviceToHost, g->stream));
+    int mat = 0;
+    if (g->lazy_blocks) CK(cudaMemcpyAsync(&mat, g->d_lazy, sizeof(int), cudaMemcpyDeviceToHost, g->stream));
     CK(cudaStreamSynchronize(g->stream));
+    g->lazy_materialised = mat;
     g->st.flow_const = sc[0];
     *energy_part = sc[0] + sc[1];
     if (g->init_timed) {
@@ -1484,16 +1512,16 @@ bool make_block_map(mgc_graph* g, const void* ptr, int dtype, CUtensorMap* out)
                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <typename E, int FN, int USE_MAX, int SPACING, int TIN = 0>
+template <typename E, int FN, int USE_MAX, int SPACING, int TIN = 0, int MODE = 0>
 int build_launch_inst(mgc_graph* g, const BuildMaps& imap, const BuildArgs& A, const BoundaryParams& P, int nz_layers)
 {
-    auto kern = k_build_tile<E, double, FN, USE_MAX, SPACING, TIN>;
+    auto kern = k_build_tile<E, double, FN, USE_MAX, SPACING, TIN, MODE>;
     const size_t smem = build_smem_bytes<E>();
     static bool attr_done = false;       // per instantiation
     if (!attr_done) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); attr_done = true; }
     const dim3 grid((unsigned)((g->L.dim[2] + BUILD_TX - 1) / BUILD_TX), (unsigned)((g->L.dim[1] + BUILD_TY - 1) / BUILD_TY), (unsigned)nz_layers);
     kern<<<grid, BUILD_THREADS, smem, g->stream>>>(g->L, g->TL, g->S, imap, A, P, g->d_flags, g->partials, g->rflag, rl(g, 0), g->pflag,
-                                                     pl(g, 0, 0), pl(g, 1, 0));
+                                                     pl(g, 0, 0), pl(g, 1, 0), g->bflag, g->d_lazy);
     g->st.kernel_launches++;
     CK(cudaGetLastError());
     return MGC_OK;
@@ -1508,16 +1536,76 @@ int build_launch(mgc_graph* g, const BuildMaps& imap, const BuildArgs& A, const 
                 // float32 image + float32 probability map + byte markers, everything staged by TMA: the compile-time variant
                 const bool fast = A.use_tma && A.prob && !A.prob_f64 && A.compute_f32 && A.tma_prob && A.tma_mark == 3 &&
                                   !A.fg_bits && !A.bg_bits && A.dbg == 0;
+                if (fast && g->lazy) {
+                    if (P.use_max) return build_launch_inst<E, 1, 1, 0, 1, 1>(g, imap, A, P, nz_layers);
+                    return build_launch_inst<E, 1, 0, 0, 1, 1>(g, imap, A, P, nz_layers);
+                }
                 if (fast) {
                     if (P.use_max) return build_launch_inst<E, 1, 1, 0, 1>(g, imap, A, P, nz_layers);
                     return build_launch_inst<E, 1, 0, 0, 1>(g, imap, A, P, nz_layers);
                 }
             }
+            if (g->lazy) FAIL(MGC_E_STATE, "internal: lazy build without its kernel variant");
             if (P.use_max) return build_launch_inst<E, 1, 1, 0>(g, imap, A, P, nz_layers);
             return build_launch_inst<E, 1, 0, 0>(g, imap, A, P, nz_layers);
         }
     }
+    if (g->lazy) FAIL(MGC_E_STATE, "internal: lazy build without its kernel variant");
     return build_launch_inst<E, -1, -1, -1>(g, imap, A, P, nz_layers);
+}
+
+// the variant a lazy build runs (build_launch: float32 image, exponential term without spacing, staged t-link inputs)
+bool lazy_variant(const BuildArgs& A, const BoundaryParams& P, int img_dtype)
+{
+    return img_dtype == MGC_F32 && P.fn == 1 && P.inv_spacing_on == 0.0 && A.use_tma && A.prob && !A.prob_f64 &&
+           A.compute_f32 && A.tma_prob && A.tma_mark == 3 && !A.fg_bits && !A.bg_bits && A.dbg == 0;
+}
+
+template <int USE_MAX>
+int lazy_list_inst(mgc_graph* g, const WorkList& tiles)
+{
+    auto kern = k_build_materialise<float, double, 1, USE_MAX, 0>;
+    const size_t smem = build_smem_bytes<float>();
+    static bool attr_done = false;
+    if (!attr_done) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); attr_done = true; }
+    kern<<<g->n_ctas * 2, BUILD_THREADS, smem, g->stream>>>(g->L, g->TL, g->S, g->lazy_maps, g->lazy_args, g->lazy_P, tiles,
+                                                           g->bflag, g->d_lazy);
+    g->st.kernel_launches++;
+    CK(cudaGetLastError());
+    return MGC_OK;
+}
+
+int lazy_materialise_list(mgc_graph* g, const WorkList& tiles)
+{
+    return g->lazy_P.use_max ? lazy_list_inst<1>(g, tiles) : lazy_list_inst<0>(g, tiles);
+}
+
+template <int USE_MAX>
+int lazy_all_inst(mgc_graph* g)
+{
+    auto kern = k_build_materialise_all<float, double, 1, USE_MAX, 0>;
+    const size_t smem = build_smem_bytes<float>();
+    static bool attr_done = false;
+    if (!attr_done) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); attr_done = true; }
+    const dim3 grid((unsigned)((g->L.dim[2] + BUILD_TX - 1) / BUILD_TX), (unsigned)((g->L.dim[1] + BUILD_TY - 1) / BUILD_TY),
+                    (unsigned)((g->L.dim[0] + BUILD_TZ - 1) / BUILD_TZ));
+    kern<<<grid, BUILD_THREADS, smem, g->stream>>>(g->L, g->TL, g->S, g->lazy_maps, g->lazy_args, g->lazy_P, g->bflag, g->d_lazy);
+    g->st.kernel_launches++;
+    CK(cudaGetLastError());
+    return MGC_OK;
+}
+
+// Every reader of cap / tr / excess outside the tile push passes (get_edge / get_trcap, further terms, the debug
+// checks, the cooperative and per-voxel solvers) sees the whole lattice: materialise what is still cold, stream-ordered,
+// and let the next upload into a staging slot wait for it.
+int lazy_materialise_all(mgc_graph* g)
+{
+    if (!g->lazy) return MGC_OK;
+    const int rc = g->lazy_P.use_max ? lazy_all_inst<1>(g) : lazy_all_inst<0>(g);
+    if (rc) return rc;
+    slots_release(g, 0x17u);
+    g->lazy = false;
+    return MGC_OK;
 }
 
 int build_launch_dtype(mgc_graph* g, int dtype, const BuildMaps& imap, const BuildArgs& A, const BoundaryParams& P, int nz_layers)
@@ -1633,6 +1721,8 @@ int mgc_reset(mgc_graph* g)
     g->st.n_voxels = n;
     g->terms_open = false;
     g->bad_pending = false;
+    g->lazy = false;
+    g->lazy_blocks = g->lazy_materialised = 0;
     return MGC_OK;
 }
 
@@ -1737,6 +1827,7 @@ int mgc_set_option(mgc_graph* g, int32_t option, int64_t value)
 {
     if (!g) return MGC_E_ARG;
     if (option == MGC_OPT_DEFER_WEIGHT_CHECK) { g->defer_check = value != 0; return MGC_OK; }
+    if (option == MGC_OPT_KEEP_INPUTS) { g->keep_inputs = value != 0; return MGC_OK; }
     FAIL(MGC_E_ARG, "unknown option");
 }
 
@@ -1769,6 +1860,7 @@ int mgc_add_regional_probability(mgc_graph* g, const mgc_array* prob, double alp
     if (prob->dtype != MGC_F32 && prob->dtype != MGC_F64) FAIL(MGC_E_ARG, "probability map must be float32 or float64");
     if (compute_dtype != MGC_F32 && compute_dtype != MGC_F64) FAIL(MGC_E_ARG, "compute dtype must be float32 or float64");
     CK(cudaSetDevice(g->device));
+    { int rcl = lazy_materialise_all(g); if (rcl) return rcl; }
     TermSpan t(g);
     const void* p = nullptr;
     int rc = stage_input(g, prob, 0, &p);
@@ -1797,6 +1889,7 @@ int mgc_add_tweights_dense(mgc_graph* g, const mgc_array* src, const mgc_array* 
     if (g->flow_started) FAIL(MGC_E_STATE, "the graph has been solved (its capacities hold residuals): reset() it before adding terms");
     if (src->dtype != MGC_F64 || snk->dtype != MGC_F64) FAIL(MGC_E_ARG, "dense t-weights must be float64");
     CK(cudaSetDevice(g->device));
+    { int rcl = lazy_materialise_all(g); if (rcl) return rcl; }
     TermSpan t(g);
     const void *ps = nullptr, *pk = nullptr;
     int rc = stage_input(g, src, 0, &ps);
@@ -1823,6 +1916,7 @@ int mgc_add_markers(mgc_graph* g, const mgc_array* fg, const mgc_array* bg)
     if (g->flow_started) FAIL(MGC_E_STATE, "the graph has been solved (its capacities hold residuals): reset() it before adding terms");
     if ((fg && fg->dtype != MGC_U8) || (bg && bg->dtype != MGC_U8)) FAIL(MGC_E_ARG, "markers must be uint8 / bool");
     CK(cudaSetDevice(g->device));
+    { int rcl = lazy_materialise_all(g); if (rcl) return rcl; }
     TermSpan t(g);
     const void *pf = nullptr, *pb = nullptr;
     int rc = MGC_OK;
@@ -1851,6 +1945,7 @@ int mgc_add_boundary(mgc_graph* g, int32_t kind, const mgc_array* image, double 
     if (kind < 0 || kind > 7) FAIL(MGC_E_ARG, "unknown boundary term");
     if (g->flow_started) FAIL(MGC_E_STATE, "the graph has been solved (its capacities hold residuals): reset() it before adding terms");
     CK(cudaSetDevice(g->device));
+    { int rcl = lazy_materialise_all(g); if (rcl) return rcl; }
     { int rc0 = check_pending(g); if (rc0) return rc0; }
     TermSpan t(g);
     const void* img = nullptr;
@@ -1994,6 +2089,17 @@ int mgc_build_voxel_graph(mgc_graph* g, const mgc_voxel_terms* t)
         }
     }
     if (const char* e = getenv("MEDPY_GC_BUILD_DBG")) A.dbg = atoi(e);
+    // lazy build: materialisation re-reads the inputs until the solve is done -- staged copies are the handle's own,
+    // caller-owned device arrays only with MGC_OPT_KEEP_INPUTS
+    const bool borrowed = d_img == t->image->data || (t->prob && d_prob == t->prob->data) || (t->fg && d_fg == t->fg->data) ||
+                          (t->bg && d_bg == t->bg->data);
+    g->lazy = g->lazy_build && !g->slab && g->bflag && (!borrowed || g->keep_inputs) && lazy_variant(A, P, t->image->dtype);
+    g->lazy_blocks = 0;
+    if (g->lazy) {
+        g->lazy_maps = imap; g->lazy_args = A; g->lazy_P = P;
+        g->lazy_blocks = (int64_t)nzt * ((g->L.dim[1] + BUILD_TY - 1) / BUILD_TY) * ((g->L.dim[2] + BUILD_TX - 1) / BUILD_TX);
+        CK(cudaMemsetAsync(g->d_lazy, 0, sizeof(int), g->stream));
+    }
 
     CK(cudaMemsetAsync(g->d_tcount, 0, 256, g->stream));
     CK(cudaMemsetAsync(g->d_flags, 0, sizeof(int), g->stream));
@@ -2086,6 +2192,7 @@ int mgc_add_nweights_dense(mgc_graph* g, int32_t axis, const mgc_array* fwd, con
     if (axis < 0 || axis >= g->user_ndim) FAIL(MGC_E_ARG, "bad axis");
     if (fwd->dtype != MGC_F64 || bwd->dtype != MGC_F64) FAIL(MGC_E_ARG, "dense n-weights must be float64");
     CK(cudaSetDevice(g->device));
+    { int rcl = lazy_materialise_all(g); if (rcl) return rcl; }
     { int rc0 = check_pending(g); if (rc0) return rc0; }
     TermSpan t(g);
     const void *pf = nullptr, *pb = nullptr;
@@ -2125,6 +2232,9 @@ int mgc_maxflow(mgc_graph* g, double* energy)
     {
         Timer t(g, &g->st.ms_solve);
         int rc = MGC_OK;
+        if (!g->use_tiles || g->use_coop || g->debug_checks) {      // no per-colour hook in these paths
+            rc = lazy_materialise_all(g); if (rc) return rc;
+        }
         if (g->use_tiles) {
             if (g->debug_checks) {
                 rc = materialise_zeros(g); if (rc) return rc;
@@ -2214,6 +2324,8 @@ int mgc_get_edge(mgc_graph* g, int64_t i, int64_t j, double* cap)
     if (i < 0 || j < 0 || i >= n || j >= n || i == j) FAIL(MGC_E_ARG, "bad node ids");
     *cap = 0.0;
     if (g->caps_fresh) return MGC_OK;
+    CK(cudaSetDevice(g->device));
+    { int rcl = lazy_materialise_all(g); if (rcl) return rcl; }
     int c[4] = {0, 0, 0, 0};
     unsigned r = (unsigned)i;
     for (int d = 0; d < g->nd; ++d) { c[d] = (int)(r / g->L.stride[d]); r %= g->L.stride[d]; }
@@ -2236,6 +2348,8 @@ int mgc_get_trcap(mgc_graph* g, int64_t node, double* trcap)
     if (!g || !trcap) return MGC_E_ARG;
     if (node < 0 || node >= (int64_t)g->L.n) FAIL(MGC_E_ARG, "node id out of range");
     if (g->tr_fresh) { *trcap = 0.0; return MGC_OK; }
+    CK(cudaSetDevice(g->device));
+    { int rcl = lazy_materialise_all(g); if (rcl) return rcl; }
     if (!g->state_init || !g->flow_started) {      // no flow yet: the net terminal capacity exactly as add_tweights left it
         CK(cudaMemcpyAsync(trcap, g->S.tr + node, sizeof(double), cudaMemcpyDeviceToHost, g->stream));
         CK(cudaStreamSynchronize(g->stream));
@@ -2278,6 +2392,14 @@ int mgc_get_stats(const mgc_graph* g, mgc_stats* out)
     if (!g || !out) return MGC_E_ARG;
     *out = g->st;
     out->device_bytes = g->device_bytes;
+    return MGC_OK;
+}
+
+int mgc_get_lazy_stats(const mgc_graph* g, int64_t* build_blocks, int64_t* materialised)
+{
+    if (!g || !build_blocks || !materialised) return MGC_E_ARG;
+    *build_blocks = g->lazy_blocks;
+    *materialised = g->lazy_materialised;
     return MGC_OK;
 }
 

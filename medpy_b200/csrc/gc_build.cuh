@@ -82,12 +82,22 @@ __device__ __forceinline__ double build_pair(const BoundaryParams& P, double a, 
 // TIN = 1: the common configuration fixed at compile time -- float32 probability map with float32 products and both
 // marker volumes as bytes, all three staged by TMA.  The generic form (TIN = 0) decides each of those per voxel with
 // warp-uniform branches: ncu's instruction mix showed ~80 of the 483 instructions per voxel going into that bookkeeping.
-template <typename E, typename T, int FN, int USE_MAX, int SPACING, int TIN = 0>
-__global__ void __launch_bounds__(BUILD_THREADS)
-k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps maps, BuildArgs A, BoundaryParams P,
-             int* __restrict__ bad, double* __restrict__ partials, int* __restrict__ rflag, WorkList rl,
-             int* __restrict__ pflag, WorkList pl0, WorkList pl1)
+// Lazy build (MODE, TIN = 1 only).  A block none of whose voxels holds source excess after the t-links (tr > 0) is COLD:
+// the max-flow phase reaches it only if flow is pushed into it, and until then the BFS, the sweeps, the relabel resets
+// and the read-out need only its rmask and height.  MODE 1 writes everything for hot blocks and only rmask, height, the
+// worklist flags and the flow-constant partial for cold ones (no exponential, 15 instead of 79 B/voxel); bflag[block]
+// says whether the cap, tr and excess planes of a block are valid.  MODE 2 materialises a cold block later: the same
+// arithmetic, but it writes only those three planes (rmask and height may have moved since) -- excess is 0 there.
+//   MODE 0: eager build (all planes, every block)    MODE 1: lazy build    MODE 2: materialise one block
+template <typename E, typename T, int FN, int USE_MAX, int SPACING, int TIN, int MODE>
+__device__ __forceinline__ void build_block(const Lattice& L, const Tiles& TL, const State<T>& S, const BuildMaps& maps,
+                                            const BuildArgs& A, const BoundaryParams& P, int* __restrict__ bad,
+                                            double* __restrict__ partials, int* __restrict__ rflag, const WorkList& rl,
+                                            int* __restrict__ pflag, const WorkList& pl0, const WorkList& pl1,
+                                            int* __restrict__ bflag, int* __restrict__ mcount, int bx, int by, int bz,
+                                            bool first, unsigned parity)
 {
+    static_assert(MODE == 0 || TIN == 1, "the lazy build exists for the staged-input variant only");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int BUILD_BX = BuildBox<E>::BX, BUILD_PAD = BuildBox<E>::PAD;
     E* s_img = reinterpret_cast<E*>(smem_raw);                                   // [10][10][BUILD_BX]
@@ -106,7 +116,9 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
 
     const int tid = threadIdx.x;
     const int lx = tid & 31, ly = tid >> 5;
-    const int x0 = blockIdx.x * BUILD_TX, y0 = blockIdx.y * BUILD_TY, z0 = (A.z_tile0 + (int)blockIdx.z) * BUILD_TZ;
+    const int x0 = bx * BUILD_TX, y0 = by * BUILD_TY, z0 = bz * BUILD_TZ;
+    const int nbx = (L.dim[2] + BUILD_TX - 1) / BUILD_TX, nby = (L.dim[1] + BUILD_TY - 1) / BUILD_TY;
+    const int blk = (bz * nby + by) * nbx + bx;
     const bool use_max = USE_MAX >= 0 ? (USE_MAX != 0) : (P.use_max != 0);
     const bool spacing = SPACING >= 0 ? (SPACING != 0) : (P.inv_spacing_on != 0.0);
 
@@ -140,6 +152,31 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
         }
         return r;
     };
+    // t-links of one voxel: add_tweights replay in the reference's order (regional, fg, bg); returns the flow-constant term
+    auto tlinks = [&](const TIn& in, T& tr) -> double {
+        double mm = 0.0;
+        if (TIN == 1) {
+            const float p = (float)in.p;
+            const float af = (float)A.alpha;
+            mm = add_tweights_dev(tr, (double)__fmul_rn(p, af), (double)__fmul_rn(__fsub_rn(1.0f, p), af));
+        } else if (A.prob) {
+            double s, t;
+            if (A.compute_f32) {
+                const float p = (float)in.p;           // exact: the map is float32 when its products are
+                const float af = (float)A.alpha;
+                s = (double)__fmul_rn(p, af);
+                t = (double)__fmul_rn(__fsub_rn(1.0f, p), af);
+            } else {
+                s = __dmul_rn(in.p, A.alpha);
+                t = __dmul_rn(__dsub_rn(1.0, in.p), A.alpha);
+            }
+            mm = add_tweights_dev(tr, s, t);
+        }
+        const bool f = (in.fb & 1u) != 0, b = (in.fb & 2u) != 0;
+        if (f) mm = __dadd_rn(mm, add_tweights_dev(tr, 65535.0, 0.0));
+        if (b) mm = __dadd_rn(mm, add_tweights_dev(tr, 0.0, 65535.0));
+        return mm;
+    };
     const bool staged_tin = TIN == 1 || (A.use_tma && ((A.prob && A.tma_prob) || A.tma_mark));
     TIn cur{0.0, 0u};
     if (!staged_tin) cur = fetch(0);          // global loads: in flight while the image block is staged
@@ -154,8 +191,12 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
     if (tid < 8) s_flags[tid] = 0;
     if (A.use_tma) {
         if (tid == 0) {
-            mbar_init(bar, 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            if (first) {
+                mbar_init(bar, 1);
+                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            } else {
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic reads of the last block are done
+            }
             const unsigned pbytes = (A.prob && A.tma_prob) ? (unsigned)(BUILD_TZ * BUILD_TY * BUILD_TX * (A.prob_f64 ? 8 : 4)) : 0u;
             const unsigned mbytes = (unsigned)(BUILD_TZ * BUILD_TY * BUILD_TX);
             mbar_expect_tx(bar, (unsigned)IMG_BYTES + pbytes + ((A.tma_mark & 1) ? mbytes : 0u) + ((A.tma_mark & 2) ? mbytes : 0u));
@@ -165,7 +206,7 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
             if (A.tma_mark & 2) tma_load_3d(s_bg, &maps.bg, bar, x0, y0, z0);
         }
         __syncthreads();
-        mbar_wait(bar, 0u);
+        mbar_wait(bar, parity);
         if (staged_tin) cur = fetch(0);
     } else {
         const E* img = reinterpret_cast<const E*>(A.img);
@@ -178,6 +219,19 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
             s_img[(hz * BUILD_HY + hy) * BUILD_BX + hx] = val;
         }
         __syncthreads();
+    }
+
+    // lazy build: the block is cold unless one of its voxels holds source excess after the t-links
+    bool cold = false;
+    if (MODE == 1) {
+        int hot = 0;
+        for (int lz = 0; lz < BUILD_TZ; ++lz) {
+            if (!(col_in && z0 + lz < L.dim[0])) continue;
+            T tr = (T)0;
+            tlinks(fetch(lz), tr);
+            if ((double)tr > 0) hot = 1;
+        }
+        cold = !__syncthreads_or(hot);
     }
 
     const bool has_py = gy + 1 < L.dim[1], has_px = gx + 1 < L.dim[2];
@@ -238,7 +292,11 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
                 return exp_term_arg(P, use_max ? fmax(a, b) : fabs(__dsub_rn(a, b)));
             };
             const double tz = arg(at(hz + 1, ly + 1, lx + 1)), ty = arg(at(hz, ly + 2, lx + 1)), tx = arg(at(hz, ly + 1, lx + 2));
-            if (__all_sync(0xffffffffu, tz <= 700.0 && ty <= 700.0 && tx <= 700.0)) {
+            if (cold && __all_sync(0xffffffffu, tz >= 0.0 && tz <= 700.0 && ty >= 0.0 && ty <= 700.0 && tx >= 0.0 && tx <= 700.0)) {
+                // a cold block keeps only the residual bits: exp_neg_inrange of an argument in [0, 700] is a positive
+                // normal number, so every valid arc of this warp is residual and no weight has to be evaluated
+                wz = 1.0; wy = 1.0; wx = 1.0;
+            } else if (__all_sync(0xffffffffu, tz <= 700.0 && ty <= 700.0 && tx <= 700.0)) {
                 wz = exp_neg_inrange(tz); wy = exp_neg_inrange(ty); wx = exp_neg_inrange(tx);
             } else {
                 wz = exp_neg(tz); wy = exp_neg(ty); wx = exp_neg(tx);
@@ -262,50 +320,35 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
             const double c0 = wz_back, c1 = wz, c3 = wy, c5 = wx;
             const double c2 = ly ? wyb[ly * 32 + lx] : s_wyh[lz * 32 + lx];
             const double c4 = lx ? wxb[ly * 33 + lx] : s_wxh[lz * 8 + ly];
-            S.cap[0][v] = (T)c0; S.cap[1][v] = (T)c1; S.cap[2][v] = (T)c2;
-            S.cap[3][v] = (T)c3; S.cap[4][v] = (T)c4; S.cap[5][v] = (T)c5;
-            // ---- t-links: add_tweights replay in the reference's order (regional, fg, bg) ----
-            T tr = (T)0;
-            double mm = 0.0;
-            if (TIN == 1) {
-                const float p = (float)cur.p;
-                const float af = (float)A.alpha;
-                mm = add_tweights_dev(tr, (double)__fmul_rn(p, af), (double)__fmul_rn(__fsub_rn(1.0f, p), af));
-            } else if (A.prob) {
-                double s, t;
-                if (A.compute_f32) {
-                    const float p = (float)cur.p;          // exact: the map is float32 when its products are
-                    const float af = (float)A.alpha;
-                    s = (double)__fmul_rn(p, af);
-                    t = (double)__fmul_rn(__fsub_rn(1.0f, p), af);
-                } else {
-                    s = __dmul_rn(cur.p, A.alpha);
-                    t = __dmul_rn(__dsub_rn(1.0, cur.p), A.alpha);
-                }
-                mm = add_tweights_dev(tr, s, t);
+            if (!cold) {
+                S.cap[0][v] = (T)c0; S.cap[1][v] = (T)c1; S.cap[2][v] = (T)c2;
+                S.cap[3][v] = (T)c3; S.cap[4][v] = (T)c4; S.cap[5][v] = (T)c5;
             }
-            const bool f = (cur.fb & 1u) != 0, b = (cur.fb & 2u) != 0;
-            if (f) mm = __dadd_rn(mm, add_tweights_dev(tr, 65535.0, 0.0));
-            if (b) mm = __dadd_rn(mm, add_tweights_dev(tr, 0.0, 65535.0));
+            T tr = (T)0;
+            const double mm = tlinks(cur, tr);
             const bool own = gz >= L.own0 && gz < L.own1;
             if (own) msum = __dadd_rn(msum, mm);
-            S.tr[v] = tr;
+            if (!cold) S.tr[v] = tr;
             // ---- solver state (same arithmetic as k_init_tile) ----
             unsigned m = (c0 > 0 ? 1u : 0u) | (c1 > 0 ? 2u : 0u) | (c2 > 0 ? 4u : 0u) | (c3 > 0 ? 8u : 0u) |
                          (c4 > 0 ? 16u : 0u) | (c5 > 0 ? 32u : 0u);
-            double out = __dadd_ru(0.0, c0);
-            out = __dadd_ru(out, c1); out = __dadd_ru(out, c2); out = __dadd_ru(out, c3);
-            out = __dadd_ru(out, c4); out = __dadd_ru(out, c5);
             const double trd = (double)tr;
             double e = 0.0;
-            if (trd > 0) { const double lim = out * SOURCE_CLAMP_SLACK; e = trd < lim ? trd : lim; if (!(out == out)) e = trd; }
+            if (!cold) {            // cold: tr <= 0 everywhere, so excess is 0 and never stored
+                double out = __dadd_ru(0.0, c0);
+                out = __dadd_ru(out, c1); out = __dadd_ru(out, c2); out = __dadd_ru(out, c3);
+                out = __dadd_ru(out, c4); out = __dadd_ru(out, c5);
+                if (trd > 0) { const double lim = out * SOURCE_CLAMP_SLACK; e = trd < lim ? trd : lim; if (!(out == out)) e = trd; }
+                if (!own) e = 0.0;
+                S.excess[v] = (T)e;
+            }
             if (trd < 0) m |= RM_SINK;
-            if (!own) e = 0.0;
-            S.excess[v] = (T)e;
-            S.rmask[v] = (uint8_t)m;
-            const int h = (own && trd < 0) ? 1 : MGC_HINF;
-            S.height[v] = h;
-            if (own && (m & 0x3fu) != 0 && h == MGC_HINF) needs_any = 1u;
+            if (MODE != 2) {
+                S.rmask[v] = (uint8_t)m;
+                const int h = (own && trd < 0) ? 1 : MGC_HINF;
+                S.height[v] = h;
+                if (own && (m & 0x3fu) != 0 && h == MGC_HINF) needs_any = 1u;
+            }
             if (e > 0) exc_any = 1u;
         }
         wz_back = wz;
@@ -313,6 +356,7 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
         // the planes of this step are read above; the next step writes the other buffer, the one after waits at its barrier
     }
 
+    if (MODE == 2) return;
     // ---- per solver tile flags and worklists (a warp row covers four 8^3 tiles: lanes 8j .. 8j+7) ----
     const unsigned bn = __ballot_sync(0xffffffffu, needs_any != 0), be = __ballot_sync(0xffffffffu, exc_any != 0);
     if (lx == 0) {
@@ -332,7 +376,11 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
         double t = s_red[0];
 #pragma unroll
         for (int w = 1; w < 8; ++w) t = __dadd_rn(t, s_red[w]);
-        partials[((A.z_tile0 + blockIdx.z) * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] = t;
+        partials[blk] = t;
+        if (MODE == 1) {
+            bflag[blk] = cold ? 0 : 1;
+            if (!cold) atomicAdd(mcount, 1);
+        }
     }
     if (tid < 4) {
         const int tx = (x0 >> 3) + tid, ty = y0 >> 3, tz = z0 >> 3;
@@ -348,6 +396,76 @@ k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps 
             }
         }
     }
+}
+
+template <typename E, typename T, int FN, int USE_MAX, int SPACING, int TIN = 0, int MODE = 0>
+__global__ void __launch_bounds__(BUILD_THREADS)
+k_build_tile(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps maps, BuildArgs A, BoundaryParams P,
+             int* __restrict__ bad, double* __restrict__ partials, int* __restrict__ rflag, WorkList rl,
+             int* __restrict__ pflag, WorkList pl0, WorkList pl1, int* __restrict__ bflag, int* __restrict__ mcount)
+{
+    build_block<E, T, FN, USE_MAX, SPACING, TIN, MODE>(L, TL, S, maps, A, P, bad, partials, rflag, rl, pflag, pl0, pl1, bflag,
+                                                       mcount, blockIdx.x, blockIdx.y, A.z_tile0 + (int)blockIdx.z, true, 0u);
+}
+
+// Materialise the cold build blocks that the push passes of one colour can reach (gc_api.cu, push_color): every tile on
+// the colour's list and each of its face neighbours -- a running tile writes flow only into those -- has its build
+// block claimed (bflag 0 -> 1, one winner) and rebuilt in MODE 2 by the CTA that claimed it.  Persistent CTAs over the
+// listed tiles; the push launch that follows on the stream sees every block complete.
+template <typename E, typename T, int FN, int USE_MAX, int SPACING>
+__global__ void __launch_bounds__(BUILD_THREADS)
+k_build_materialise(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps maps, BuildArgs A, BoundaryParams P,
+                    WorkList tiles, int* __restrict__ bflag, int* __restrict__ mcount)
+{
+    __shared__ int s_claim[8];
+    __shared__ int s_n;
+    const int n = *(volatile int*)tiles.count;
+    const int nbx = (L.dim[2] + BUILD_TX - 1) / BUILD_TX, nby = (L.dim[1] + BUILD_TY - 1) / BUILD_TY;
+    unsigned done = 0;                                   // blocks this CTA built so far (mbarrier phase)
+    for (int i = blockIdx.x; i < n; i += gridDim.x) {
+        const int t = tiles.items[i];
+        if (threadIdx.x == 0) s_n = 0;
+        __syncthreads();
+        if (threadIdx.x < 7) {
+            const int tx = t % TL.nt[2], r = t / TL.nt[2], ty = r % TL.nt[1], tz = r / TL.nt[1];
+            const int k = threadIdx.x;           // 0..5: face neighbour across face k, 6: the tile itself
+            int z = tz, y = ty, x = tx;
+            if (k < 6) {
+                const int d = (k & 1) ? 1 : -1;
+                if ((k >> 1) == 0) z += d; else if ((k >> 1) == 1) y += d; else x += d;
+            }
+            if (z >= 0 && y >= 0 && x >= 0 && z < TL.nt[0] && y < TL.nt[1] && x < TL.nt[2]) {
+                const int b = (z * nby + y) * nbx + (x >> 2);
+                if (*(volatile int*)(bflag + b) == 0 && atomicCAS(bflag + b, 0, 1) == 0) {
+                    s_claim[atomicAdd(&s_n, 1)] = b;
+                    atomicAdd(mcount, 1);
+                }
+            }
+        }
+        __syncthreads();
+        const int nc = s_n;
+        for (int j = 0; j < nc; ++j) {
+            const int b = s_claim[j];
+            build_block<E, T, FN, USE_MAX, SPACING, 1, 2>(L, TL, S, maps, A, P, nullptr, nullptr, nullptr, WorkList{}, nullptr,
+                                                          WorkList{}, WorkList{}, nullptr, nullptr, b % nbx, (b / nbx) % nby,
+                                                          b / (nbx * nby), done == 0, done & 1u);
+            ++done;
+            __syncthreads();                     // staged inputs and weight planes are free for the next block
+        }
+    }
+}
+
+// Materialise every block that is still cold (readers that need the whole lattice): one CTA per build block.
+template <typename E, typename T, int FN, int USE_MAX, int SPACING>
+__global__ void __launch_bounds__(BUILD_THREADS)
+k_build_materialise_all(Lattice L, Tiles TL, State<T> S, const __grid_constant__ BuildMaps maps, BuildArgs A, BoundaryParams P,
+                        int* __restrict__ bflag, int* __restrict__ mcount)
+{
+    const int blk = ((int)blockIdx.z * (int)gridDim.y + (int)blockIdx.y) * (int)gridDim.x + (int)blockIdx.x;
+    if (bflag[blk]) return;
+    build_block<E, T, FN, USE_MAX, SPACING, 1, 2>(L, TL, S, maps, A, P, nullptr, nullptr, nullptr, WorkList{}, nullptr, WorkList{},
+                                                  WorkList{}, nullptr, nullptr, blockIdx.x, blockIdx.y, blockIdx.z, true, 0u);
+    if (threadIdx.x == 0) { bflag[blk] = 1; atomicAdd(mcount, 1); }
 }
 
 template <typename E>

@@ -267,6 +267,9 @@ public:
         d["ms_terms"] = s.ms_terms; d["ms_solve"] = s.ms_solve; d["ms_readout"] = s.ms_readout;
         d["ms_push"] = s.ms_push; d["ms_relabel"] = s.ms_relabel; d["ms_boundary"] = s.ms_boundary; d["ms_init"] = s.ms_init;
         d["flow_const"] = s.flow_const; d["energy"] = s.energy; d["device_bytes"] = s.device_bytes;
+        int64_t bb = 0, bm = 0;
+        check(mgc_get_lazy_stats(g_, &bb, &bm), g_);
+        d["build_blocks"] = bb; d["blocks_materialised"] = bm;
         return d;
     }
     // ---- z-slab stepping (device pointers as integers, e.g. torch.Tensor.data_ptr()) ----
@@ -559,6 +562,7 @@ PYBIND11_MODULE(_mgc, m)
     m.attr("SOURCE") = MGC_SOURCE;
     m.attr("SINK") = MGC_SINK;
     m.attr("OPT_DEFER_WEIGHT_CHECK") = MGC_OPT_DEFER_WEIGHT_CHECK;
+    m.attr("OPT_KEEP_INPUTS") = MGC_OPT_KEEP_INPUTS;
     m.attr("LABELS_ADJACENCY") = MGC_LABELS_ADJACENCY;
     m.attr("LABELS_STAWIASKI") = MGC_LABELS_STAWIASKI;
     m.attr("LABELS_STAWIASKI_DIRECTED") = MGC_LABELS_STAWIASKI_DIRECTED;

@@ -24,6 +24,11 @@ def _as_u8(t):
     return t
 
 
+def _keep_inputs_option():
+    from .. import _lib
+    return _lib._mgc.OPT_KEEP_INPUTS
+
+
 def graph_from_device_arrays(fg_markers, bg_markers, image=None, boundary=None, sigma=None, spacing=False,
                              prob=None, alpha=None, graph=None, stream=None):
     """Build (or rebuild into ``graph``) the lattice graph from device arrays.
@@ -48,6 +53,10 @@ def graph_from_device_arrays(fg_markers, bg_markers, image=None, boundary=None, 
     # one native call: single-pass fused build on 1-D..3-D lattices (mgc_build_voxel_graph), the per-term kernels in
     # the reference's order otherwise.  A non-positive n-link weight is reported by maxflow() (ValueError).
     graph.defer_weight_check(True)
+    # the inputs stay referenced by the graph until its next build or reset, so the build may run lazily on them
+    # (cold blocks are built again from these arrays when the solve reaches them)
+    nat.set_option(_keep_inputs_option(), 1)
+    graph._inputs = (fg_markers, bg_markers, image, prob)
     compute_f32 = prob is not None and "float32" in str(prob.dtype)
     kind = _KINDS[boundary] if boundary is not None else -1
     sp = [float(s) for s in spacing] if spacing else None

@@ -76,6 +76,7 @@ class GraphDouble:
         # in ONE native call (mgc_build_voxel_graph: single-pass fused build) when the markers arrive or anything else
         # needs the graph.  Only while nothing has reached the device yet (_fresh).
         self._lazy = None
+        self._inputs = None
         self._fresh = True
         if sparse:
             if self._journal is None:
@@ -415,6 +416,7 @@ class GraphDouble:
         self._pending = []
         self._lazy = None
         self._fresh = True
+        self._inputs = None         # device arrays a lazy build may still read (graph_from_device_arrays)
         if self._native is not None:
             self._native.reset()
 
